@@ -22,6 +22,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 FLOP_PER_IMAGE_FWD_BWD = 105_382_969_344  # BASELINE.md section 2 (GEMM-only, 3x forward)
 CLIP_FLOP_PER_PAIR_FWD_BWD = 3 * 14_780_000_000  # SURVEY.md 8a row a16: 14.78 GFLOP / pair forward (vision 8.82 + text 5.96)
@@ -332,6 +333,31 @@ def eager_gpu_leg(rank, world, dev, steps, warmup):
 
 
 # ------------------------------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step handed its caller, for output-for-output comparison of two builds
+# ------------------------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 21  # values kept per dumped array (8 MB in float32); at most 6 arrays -> under 64 MB in all
+
+
+def dump_outputs(out_dir, loss, arenas):
+    """Writes ``loss.npy`` (the step's loss) and, per parameter arena ``name``, ``<name>params.npy`` (the parameters after the
+    step's Adam update) and ``<name>grads.npy`` (the step's gradients), all float32.  An arena longer than DUMP_SAMPLE is
+    cut to DUMP_SAMPLE values at positions drawn from a fixed seed, the same positions on every run."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().reshape(1)}
+    for name, a in arenas:
+        arrays[f"{name}params"], arrays[f"{name}grads"] = a.flat, a.grad
+    for name, t in arrays.items():
+        t = t.detach().reshape(-1)
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t[idx.to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
+
+
+# ------------------------------------------------------------------------------------------------------------------
 # the B200 arm
 # ------------------------------------------------------------------------------------------------------------------
 def run_b200(args):
@@ -453,6 +479,8 @@ def run_b200(args):
     final_loss = loss.item()
     if not (final_loss == final_loss and abs(final_loss) < 1e4):
         raise SystemExit(f"bench.py: loss diverged ({final_loss})")
+    if args.dump_outputs and rank == 0:  # before the end-to-end steps below move the parameters on
+        dump_outputs(args.dump_outputs, loss, zip(("vit_", "text_", "glue_"), model.arenas()) if is_clip else [("", model.arena)])
 
     dog.enter("end-to-end steps")
     # ---- end to end: pinned host batches -> H2D on a copy stream (prefetched one step ahead) -> step -> loss D2H --
@@ -659,7 +687,11 @@ def main():
                          "graph; torch = torch.distributed, one all-reduce behind the graph (round 1's schedule); auto = graph for N <= 2, "
                          "flat for N >= 3 (measured: graph 0.990 at N = 2 but 0.894 at N = 8, DESIGN.md section 4)")
     ap.add_argument("--no-eager-baseline", action="store_true", help="skip the PyTorch-eager-on-GPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss, updated parameters and gradients to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.dp_mode == "auto":
         args.dp_mode = "graph" if int(os.environ.get("WORLD_SIZE", "1")) <= 2 else "flat"
     args.flat_allreduce = args.dp_mode in ("flat", "torch")
